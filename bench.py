@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — forward+adjoint stencil throughput (BASELINE.json metric) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2|c4|c5] [--dump-outputs DIR]
 
 One "step" = one forward kernel + one adjoint kernel over the whole field (per GPU: weak scaling, every rank owns
 a slab of the workload's full single-GPU shape; ghost planes are exchanged with the neighbours before each kernel
@@ -9,17 +9,25 @@ when N > 1).  Prints ONE JSON line on rank 0.  The headline workload is C3 (the 
 1/2/4/8 GPUs); at N = 1 the same line carries the other named configurations (``workloads``: C2, C4, C5, each with its own
 timed region, roofline and clocks), the ``torch.autograd.Function`` path (``function_path``), full-size parity against the
 CPU oracle (``parity``) and the end-to-end legs with host buffers (``e2e``, ``e2e_plugin``).  See DESIGN.md "Measurement".
+
+The benchmark writes nothing into the source tree, which may be read-only: kernels it has to compile at run time (NVRTC
+cubins, the oracle's C kernels) go to a temporary directory that is removed at exit; the cubins build() compiled into the
+tree are used from there.
 """
 import argparse
+import atexit
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True
 
 METRIC = 'forward+adjoint Mcell-updates/s'
 UNIT = 'Mcell-updates/s'
@@ -39,6 +47,7 @@ TOL = {'f32': 1e-6, 'f64': 1e-12}          # north_star: <= 1e-6 relative in fp3
 # double: AutoDiffOp(..., data_type='double') reproduces it and is checked at 1e-6 beside this (``double_arithmetic``).
 TOL_OVERRIDE = {('c5', 'adjoint'): 1e-5}
 BAD_CLOCK_REASONS = {'hw_slowdown', 'hw_thermal_slowdown', 'sw_thermal_slowdown'}
+DUMP_BYTES = 60 * 10**6          # --dump-outputs: payload of all arrays together, under 64 MB with the .npy headers
 
 
 def parse_args():
@@ -60,7 +69,32 @@ def parse_args():
     ap.add_argument('--no-e2e', action='store_true', help='skip the end-to-end leg (diagnostic runs)')
     ap.add_argument('--only-headline', action='store_true', help='skip the extra N = 1 legs (workloads, function path, parity)')
     ap.add_argument('--cpu-shape', type=int, nargs='*', default=None, help='CPU arm: sample shape (default: the full workload)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last one computed (the forward outputs and the input '
+                         'gradients of the headline workload) as DIR/<field>.npy; arrays over %d MB in all are replaced '
+                         'by a fixed seeded sample of their elements' % (DUMP_BYTES // 10**6))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes what the GPU path computed: it needs --impl ours')
+    return args
+
+
+def use_private_build_dirs():
+    """Kernels compiled at run time go to a temporary directory, removed at exit (see the module docstring).  The cubins
+    build() left in the package's cache are linked into the temporary cache, so they are not compiled again."""
+    tmp = tempfile.mkdtemp(prefix='psad_bench_')
+    atexit.register(shutil.rmtree, tmp, True)
+    if 'PSAD_CACHE_DIR' not in os.environ:
+        cubins = os.path.join(tmp, 'cubin')
+        os.makedirs(cubins)
+        built = os.path.join(ROOT, 'pystencils_autodiff_b200', '_cubin_cache')
+        for name in (os.listdir(built) if os.path.isdir(built) else []):
+            if name.endswith('.cubin'):
+                os.symlink(os.path.join(built, name), os.path.join(cubins, name))
+        os.environ['PSAD_CACHE_DIR'] = cubins
+    os.environ.setdefault('PSAD_ORACLE_BUILD_DIR', os.path.join(tmp, 'oracle'))
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -402,6 +436,29 @@ def measure_resident(env, wl, shape, steps, warmup, cooldown_s=0.0, halo='auto')
     return res, slab, op
 
 
+def dump_outputs(env, op, slab, out_dir):
+    """``--dump-outputs``: the arrays the timed step hands its caller — the forward outputs and the adjoint's input
+    gradients of this rank's slab — as ``out_dir/<field>.npy`` in their own dtype (``<field>.rank<r>.npy`` when N > 1).
+    Every rank gets DUMP_BYTES / N: when its arrays exceed that together, each is replaced by its elements at the same
+    seeded, sorted flat indices in every run (``numpy.random.default_rng(0)``), so that two builds of the project can be
+    compared output for output."""
+    import numpy as np
+    torch = env.torch
+    names = list(dict.fromkeys(f.name for f in list(op.forward_output_fields) + list(op.backward_output_fields)))
+    arrays = {n: slab.dh.owned(n) for n in names}
+    budget = DUMP_BYTES // env.world
+    sample = sum(t.numel() * t.element_size() for t in arrays.values()) > budget
+    suffix = '.rank%d' % env.rank if env.world > 1 else ''
+    os.makedirs(out_dir, exist_ok=True)
+    torch.cuda.synchronize()
+    for name, t in arrays.items():
+        if sample:
+            k = budget // len(arrays) // t.element_size()
+            idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), size=k))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, name + suffix + '.npy'), t.cpu().numpy())
+
+
 def function_path(env, op, slab, steps):
     """The path the north-star names: ``Function.apply`` + backward on RESIDENT tensors — output and gradient allocation
     (``torch.empty``), ``save_for_backward``, the autograd engine and the ctypes call all inside the timed region —
@@ -723,6 +780,8 @@ def main_ours(args):
         shape = (shape[0] // env.world,) + shape[1:]
     n_launch0 = runtime.launch_count()
     head, slab, op = measure_resident(env, wl, shape, args.steps, args.warmup, halo=args.halo)
+    if args.dump_outputs:
+        dump_outputs(env, op, slab, args.dump_outputs)     # before the legs below overwrite the arrays
     cells = int(np.prod(shape))
 
     legs = {}
@@ -836,4 +895,5 @@ def main_ours(args):
 
 if __name__ == '__main__':
     a = parse_args()
+    use_private_build_dirs()
     sys.exit(main_reference(a) if a.impl == 'reference' else main_ours(a))

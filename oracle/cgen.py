@@ -25,7 +25,8 @@ from sympy.printing.c import C99CodePrinter
 
 from ._model import as_collection, field_dtype, ghost_width, is_access, offsets_of
 
-_BUILD_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), '_build')
+# $PSAD_ORACLE_BUILD_DIR: compile outside the tree (bench.py uses a temporary directory: the tree may be read-only)
+_BUILD_DIR = os.environ.get('PSAD_ORACLE_BUILD_DIR') or os.path.join(os.path.dirname(os.path.abspath(__file__)), '_build')
 _CTYPES = {np.dtype(np.float32): 'float', np.dtype(np.float64): 'double'}
 
 FLAGS = {
