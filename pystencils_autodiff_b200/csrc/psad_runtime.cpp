@@ -77,7 +77,7 @@ enum { CU_DEVICE_ATTRIBUTE_MULTIPROCESSOR_COUNT = 16, CU_DEVICE_ATTRIBUTE_COMPUT
        CU_DEVICE_ATTRIBUTE_COMPUTE_CAPABILITY_MINOR = 76, CU_DEVICE_ATTRIBUTE_MAX_SHARED_MEMORY_PER_BLOCK_OPTIN = 97 };
 enum { CU_FUNC_ATTRIBUTE_SHARED_SIZE_BYTES = 1, CU_FUNC_ATTRIBUTE_LOCAL_SIZE_BYTES = 3, CU_FUNC_ATTRIBUTE_NUM_REGS = 4,
        CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES = 8 };
-enum { CU_TENSOR_MAP_DATA_TYPE_FLOAT32 = 7, CU_TENSOR_MAP_DATA_TYPE_FLOAT64 = 8 };
+enum { CU_TENSOR_MAP_DATA_TYPE_FLOAT16 = 6, CU_TENSOR_MAP_DATA_TYPE_FLOAT32 = 7, CU_TENSOR_MAP_DATA_TYPE_FLOAT64 = 8 };
 
 struct Driver {
   void* lib = nullptr;
@@ -560,7 +560,8 @@ static int build_args(const psad_plan_t& P, const char* kname, int sm_count, int
       if (((uintptr_t)A.ptr[f]) % 16 != 0) return fail(PSAD_ERR_INVALID, "%s: field %d pointer is not 16-byte aligned", kname, f);
       if ((A.stride[f][1] * fp.elem_size) % 16 != 0 || (nd == 3 && (A.stride[f][0] * fp.elem_size) % 16 != 0))
         return fail(PSAD_ERR_INVALID, "%s: field %d row/plane pitch is not a multiple of 16 bytes", kname, f);
-      if (fp.tma && fp.elem_size != 4 && fp.elem_size != 8) return fail(PSAD_ERR_INVALID, "TMA fields must be float32/float64");
+      if (fp.tma && fp.elem_size != 2 && fp.elem_size != 4 && fp.elem_size != 8)
+        return fail(PSAD_ERR_INVALID, "TMA fields must be float16/float32/float64");
     }
   } else {
     return fail(PSAD_ERR_INVALID, "unknown kernel kind %d", P.kind);
@@ -644,7 +645,9 @@ static int encode_one_map(const psad_plan_t& P, const psad_field_plan_t& fp, voi
   unsigned estr[3] = {1, 1, 1};
   for (int d = 0; d < nd; ++d)
     if (box[d] < 1 || box[d] > 256) return fail(PSAD_ERR_INVALID, "TMA box dim %d = %u out of range", d, box[d]);
-  CUresult r = g_drv.cuTensorMapEncodeTiled(out, fp.elem_size == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT64,
+  const int dtype = fp.elem_size == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16
+                    : fp.elem_size == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT64;
+  CUresult r = g_drv.cuTensorMapEncodeTiled(out, dtype,
                                             (unsigned)nd, base, gdim, gstr, box, estr,
                                             /*interleave none*/ 0, /*swizzle none*/ 0, /*L2 promotion*/ l2promo, /*oob fill: zeros*/ 0);
   if (r != 0) return cu_fail(r, "cuTensorMapEncodeTiled");

@@ -510,6 +510,8 @@ class SlabDataHandling:
         self._ev_halo = None
         # peer halos: the stencil kernels read their ghost planes from the neighbouring GPUs' arrays (CUDA IPC mappings,
         # NVLink) instead of having them exchanged first — see _PeerHalo
+        # float16 arrays always take the NCCL exchange: the peer-halo kernel instance is not built for them
+        self._peer_forced = peer_halo is True
         if peer_halo == 'auto':
             peer_halo = peer_halos_pay_off(self.dec.local_shape, self.dec.world_size, backend, self.device)
         if peer_halo and periodic:
@@ -552,7 +554,12 @@ class SlabDataHandling:
         else:
             shape = self.dec.local_shape
         arr = self.torch.zeros(shape + tail, dtype=numpy_dtype_to_torch(dtype), device=self.device)
-        if self.peer is not None and name not in self._replicated:
+        if self.peer is not None and np.dtype(dtype) == np.float16 and name not in self._replicated:
+            if self._peer_forced:
+                raise ValueError('peer halos are not available for float16 arrays (peer_halo=False or \'auto\' exchange '
+                                 'their ghost planes through NCCL)')
+            # 'auto': not registered, so every launch on this array takes the NCCL exchange (_PeerHalo.applies)
+        elif self.peer is not None and name not in self._replicated:
             self.peer.register(arr)              # collective: every rank adds its arrays in the same order
         self.gpu_arrays[name] = arr
         self.fields[name] = Field.create_fixed_size(name, shape + tail, index_dimensions=len(tail), dtype=dtype)

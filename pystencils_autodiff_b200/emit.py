@@ -30,7 +30,12 @@ from .linopt import plan_linear
 KERNEL_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'csrc', 'kernels')
 EMITTER_VERSION = '19'
 
-_CT = {np.dtype(np.float32): 'float', np.dtype(np.float64): 'double'}
+_CT = {np.dtype(np.float16): 'psad_half', np.dtype(np.float32): 'float', np.dtype(np.float64): 'double'}
+_F16 = np.dtype(np.float16)
+# float16 fields: storage type psad_half (psad_half.cuh), values converted to fp32 where they enter the registers
+HALF_HEADER = 'psad_half.cuh'
+# headers that only some kernels include: hashed into the cache key of those kernels only
+_OPTIONAL_HEADERS = (HALF_HEADER,)
 # AutoDiffOp(..., fast_math=True): denormals flushed, approximate reciprocal / square root (2 ulp); the explicit FMA
 # chains stay as they are
 FAST_MATH_OPTIONS = ['-ftz=true', '-prec-div=false', '-prec-sqrt=false']
@@ -55,6 +60,8 @@ class EmittedKernel:
         h.update(self.source.encode())
         h.update(' '.join(self.options).encode())
         for fn in sorted(os.listdir(KERNEL_DIR)):
+            if fn in _OPTIONAL_HEADERS and ('#include "%s"' % fn) not in self.source:
+                continue
             with open(os.path.join(KERNEL_DIR, fn), 'rb') as fh:
                 h.update(fh.read())
         return '%s_%s' % (self.name[:40], h.hexdigest())
@@ -239,7 +246,10 @@ def emit_generic(ir: StencilKernelIR, threads=256) -> EmittedKernel:
     lz, ly, lx = _off3(ir.lhs_offset)
 
     L = _header(ir, 'generic')
-    L += ['#include "psad_common.cuh"', '', 'typedef %s CT;' % CT]
+    L += ['#include "psad_common.cuh"']
+    if any(f.dtype.numpy_dtype == _F16 for f in fields):
+        L.append('#include "%s"' % HALF_HEADER)
+    L += ['', 'typedef %s CT;' % CT]
     for f in fields:
         L.append('typedef %s T_%d;  // %s' % (_CT[f.dtype.numpy_dtype], fidx[f.name], f.name))
     L += ['',
@@ -363,8 +373,10 @@ def march_ineligible_reason(ir: StencilKernelIR) -> Optional[str]:
     for f in ir.all_fields:
         if f.index_dimensions:
             return 'index dimensions'
-        if f.dtype.numpy_dtype not in (np.dtype(np.float32), np.dtype(np.float64)):
-            return 'only float32/float64 fields'
+        if f.dtype.numpy_dtype not in (_F16, np.dtype(np.float32), np.dtype(np.float64)):
+            return 'only float16/float32/float64 fields'
+    if len({f.dtype.numpy_dtype for f in ir.all_fields}) > 1 and any(f.dtype.numpy_dtype == _F16 for f in ir.all_fields):
+        return 'float16 fields mixed with wider fields'
     if not ir.input_fields:
         return 'no input fields'
     for f in ir.input_fields:
@@ -420,10 +432,20 @@ def _emit_march(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, maske
     scalars = [s.name for s in ir.scalars]
     nd = ir.ndim
     max_esize = max(f.dtype.itemsize for f in fields)
+    half = max_esize == 2     # all fields float16 (march_ineligible_reason): 8-byte vectors of 4 halves, fp32 window
+
+    def vec_cells(es):       # cells per shared load / global store vector
+        return 4 if es == 2 else 16 // es
+
+    def reg_type(f):         # type of an output field's results in registers (rounded to fp16 only by the store)
+        return CT if f.dtype.itemsize == 2 else _CT[f.dtype.numpy_dtype]
 
     # ---- geometry ------------------------------------------------------------------------------------------
-    SX = t.sx or 4   # cells per thread along x: one 16-byte vector for 4-byte types, two for 8-byte types
-    if (SX * min(f.dtype.itemsize for f in fields)) % 16:
+    SX = t.sx or 4   # cells per thread along x: one 16-byte vector for 4-byte types, two for 8-byte types, one 8-byte
+    #                  vector for float16 (8 halves per lane would make the box 256 + pads wide: over the TMA limit)
+    if half and SX % 4:
+        raise ValueError('sx must be a multiple of 4 for float16 fields')
+    if not half and (SX * min(f.dtype.itemsize for f in fields)) % 16:
         raise ValueError('sx*itemsize must be a multiple of 16 bytes')
     TX = 32 * SX
     mh = ir.max_halo                        # per ndim axis (lo, hi)
@@ -433,11 +455,12 @@ def _emit_march(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, maske
     # measured on B200 (scripts/sweep.py, profiles/): fp32 3-D 32x128 tiles / 2 rows per thread, fp32 2-D 16x128 / 1 row,
     # fp64 21x128 tiles / 3 rows, x-halos by warp shuffle (27-pt: 6.44 TB/s)
     cross_cse = _is_nonlinear(ir) if t.cross_cse is None else bool(t.cross_cse)
-    if max_esize == 4:
+    if max_esize <= 4:
         RY = t.ry or (2 if nd == 3 else 1)
         # cross-cell CSE keeps the shared temporaries of all the thread's cells live: 15+1 warps (128 registers) instead
         # of 16+1 (96) — TV-gradient adjoint 0.758 -> 0.722 ms, and 1.00 ms when it has to spill
-        TY = t.ty or ((30 if cross_cse else 32) if nd == 3 else 16)
+        # float16: the conversions take the 15+1-warp CSE tile over 128 registers (36 bytes spilled); 11+1 warps fit
+        TY = t.ty or (((22 if half else 30) if cross_cse else 32) if nd == 3 else 16)
     else:
         # 7 consumer warps + the producer warp = 8 warps: ptxas budgets registers for the CTA size rounded up to 4
         # warps, so 8+1 warps would be capped at 168 registers and spill (the 27-point window needs ~240)
@@ -455,19 +478,21 @@ def _emit_march(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, maske
     for ti, f in enumerate(tma_fields):
         h3 = [(0, 0)] * (3 - nd) + list(ir.halo(f.name))
         es = f.dtype.itemsize
-        vec = 16 // es
+        vec = vec_cells(es)
+        pad = 16 // es       # pads in whole 16-byte units: box rows stay a multiple of 16 bytes, lane loads aligned
         hxl, hxr = h3[2]
         if hxl > SX or hxr > SX:
             raise ValueError('x halo wider than the per-thread strip')
-        padl = -(-hxl // vec) * vec
-        padr = -(-hxr // vec) * vec
+        padl = -(-hxl // pad) * pad
+        padr = -(-hxr // pad) * pad
         boxw = TX + padl + padr
         boxh = TY + h3[1][0] + h3[1][1]
         if boxw > 256 or boxh > 256:
             raise ValueError('TMA box too large')
         nbytes = boxw * boxh * es
         geo[f.name] = dict(ti=ti, es=es, vec=vec, nv=SX // vec, hz=h3[0], hy=h3[1], hx=h3[2], padl=padl, boxw=boxw,
-                           boxh=boxh, bytes=nbytes, off=off, T=_CT[f.dtype.numpy_dtype])
+                           boxh=boxh, bytes=nbytes, off=off, T=_CT[f.dtype.numpy_dtype],
+                           Tw='float' if es == 2 else _CT[f.dtype.numpy_dtype], ww=max(1, es // 4))   # window: fp16 as float
         off += -(-nbytes // 128) * 128
     STAGE_BYTES = off
     # ---- plane partial sums --------------------------------------------------------------------------------------
@@ -569,8 +594,8 @@ def _emit_march(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, maske
     # register budget: window elements + outputs + addressing; decides how many CTAs we ask ptxas to fit per SM
     words = sum(len({(u[1], c) for u in held[f.name][j] for c in
                      (range(u[2] * geo[f.name]['vec'], (u[2] + 1) * geo[f.name]['vec']) if u[0] == 'U' else [u[2]])})
-                * (geo[f.name]['es'] // 4) for f in tma_fields for j in range(D + 1))
-    words += sum(SX * (lhs.field.dtype.itemsize // 4) for lhs, _ in ir.main)
+                * geo[f.name]['ww'] for f in tma_fields for j in range(D + 1))
+    words += sum(SX * (np.dtype(ir.compute_dtype).itemsize if half else lhs.field.dtype.itemsize) // 4 for lhs, _ in ir.main)
     words += sum((qc['hi'] - qc['lo'] + 1) * RY * SX * (np.dtype(ir.compute_dtype).itemsize // 4) for qc in q_classes)
     est_regs = min(255, words + 48)
     # ptxas budgets registers for the CTA size rounded up to 4 warps; a tile whose window cannot fit would spill
@@ -598,7 +623,7 @@ def _emit_march(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, maske
     # ---- source -------------------------------------------------------------------------------------------------
     jrel = min([j for j in range(D + 1) if any(fresh[f.name][j] for f in tma_fields)] or [D])
     # ring = planes still read from shared memory (D - jrel + 1) + `lookahead` planes in flight ahead of them
-    lookahead = t.lookahead or (3 if max_esize == 4 else 4)   # measured optima (fp32 3-D: sharp at 3; fp64 27-pt: 4)
+    lookahead = t.lookahead or (3 if max_esize <= 4 else 4)   # measured optima (fp32 3-D: sharp at 3; fp64 27-pt: 4)
     STAGES = t.stages or (D - jrel + 1 + max(1, lookahead))
     if STAGES < D - jrel + 2:
         raise ValueError('ring too small')
@@ -610,7 +635,8 @@ def _emit_march(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, maske
     L = _header(ir, 'march')
     if t.store_mode != 1:
         L.append('#define PSAD_STORE_MODE %d' % t.store_mode)
-    L += ['#include "psad_common.cuh"', '', 'typedef %s CT;' % CT, 'namespace cfg {',
+    L += ['#include "psad_common.cuh"'] + (['#include "%s"' % HALF_HEADER] if half else [])
+    L += ['', 'typedef %s CT;' % CT, 'namespace cfg {',
           'constexpr int NDIM = %d, TX = %d, TY = %d, TXS = %d, XORG = 0, TYS = %d, YORG = 0;' % (nd, TX, TY, TX, TY),
           'constexpr int THREADS = %d, MIN_CTAS = %d, STAGES = %d, HZL = %d, HZH = %d, JREL = %d, NP = %d;'
           % (THREADS, min_ctas, STAGES, HZL, HZH, jrel, NP),
@@ -629,11 +655,11 @@ def _emit_march(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, maske
             all_rows = sorted({u[1] for j in range(D + 1) for u in held[f.name][j]})
             for k in range(NP):
                 for row in all_rows:
-                    L.append('  %s f%d_k%d_r%d[%d];  // %s, window slot %d, row %+d' % (g['T'], g['ti'], k, row + g['hy'][0], W,
+                    L.append('  %s f%d_k%d_r%d[%d];  // %s, window slot %d, row %+d' % (g['Tw'], g['ti'], k, row + g['hy'][0], W,
                                                                                      f.name, k, row))
         else:
             for j, row in sorted({(j, u[1]) for j in range(D + 1) for u in held[f.name][j]}):
-                L.append('  %s f%d_k%d_r%d[%d];  // %s, plane %+d, row %+d' % (g['T'], g['ti'], j, row + g['hy'][0], W, f.name,
+                L.append('  %s f%d_k%d_r%d[%d];  // %s, plane %+d, row %+d' % (g['Tw'], g['ti'], j, row + g['hy'][0], W, f.name,
                                                                             j - HZL, row))
     for ci, qc in enumerate(q_classes):
         for k in range(D + 1):
@@ -703,7 +729,10 @@ def _emit_march(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, maske
                         L.append('  psad_lds_pair<%s>(%s, lane_hi, &%s);' % (g['T'], rp, elem(f, j, row, 0)))
                         own = []
                     for u in own:
-                        L.append('  psad_lds_vec<%s>(%s + %d, &%s);' % (g['T'], rp, u[2] * g['vec'], elem(f, j, row, u[2] * g['vec'])))
+                        if g['es'] == 2:
+                            L.append('  psad_lds_h4(%s + %d, &%s);' % (rp, u[2] * g['vec'], elem(f, j, row, u[2] * g['vec'])))
+                        else:
+                            L.append('  psad_lds_vec<%s>(%s + %d, &%s);' % (g['T'], rp, u[2] * g['vec'], elem(f, j, row, u[2] * g['vec'])))
                     for u in sorted(x for x in fr if x[0] == 'H' and x[1] == row):
                         c = u[2]
                         if t.shuffle:
@@ -819,11 +848,11 @@ def _emit_march(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, maske
             if masked:
                 L.append('      const unsigned m = ((zm >> %d) & 1u) ? R.xmask : 0u;' % r)
             for lhs, _ in ir.main:
-                L.append('      %s o%d[%d];' % (_CT[lhs.field.dtype.numpy_dtype], fidx[lhs.field.name], SX))
+                L.append('      %s o%d[%d];' % (reg_type(lhs.field), fidx[lhs.field.name], SX))
             for c in range(SX):
                 if shared is not None:
                     for lhs, _ in main_exprs:
-                        To = _CT[lhs.field.dtype.numpy_dtype]
+                        To = reg_type(lhs.field)
                         fi = fidx[lhs.field.name]
                         if masked:
                             L.append('      o%d[%d] = ((m >> %d) & 1u) ? (%s)(%s) : (%s)0;' % (fi, c, c, To, shared[(fi, r, c)], To))
@@ -836,7 +865,7 @@ def _emit_march(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, maske
                     L.append('        const CT %s = %s;' % (_c_ident(lhs.name), pr.print_with(rhs.xreplace(subs), local)))
                     local[lhs] = _c_ident(lhs.name)
                 for lhs, rhs in main_exprs:
-                    To = _CT[lhs.field.dtype.numpy_dtype]
+                    To = reg_type(lhs.field)
                     text = pr.print_with(rhs.xreplace(subs), local)
                     if masked:
                         L.append('        o%d[%d] = ((m >> %d) & 1u) ? (%s)(%s) : (%s)0;' % (fidx[lhs.field.name], c, c, To, text, To))
@@ -846,12 +875,13 @@ def _emit_march(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, maske
             for f in out_fields:
                 fi = fidx[f.name]
                 To = _CT[f.dtype.numpy_dtype]
-                vec = 16 // f.dtype.itemsize
+                vec = vec_cells(f.dtype.itemsize)
                 zterm = ' + (long long)z * A.stride[%d][0]' % fi if nd == 3 else ''
                 L.append('      %s* q%d = R.o%d%s + %d * A.stride[%d][1];' % (To, fi, fi, zterm, r, fi))
+                store = 'psad_stg_h4' if f.dtype.itemsize == 2 else 'psad_stg_vec<%s>' % To
                 for v in range(SX // vec):
-                    L.append('      if (R.xs + %d <= (int)A.shape[2]) psad_stg_vec<%s>(q%d + %d, &o%d[%d]);'
-                             % ((v + 1) * vec, To, fi, v * vec, fi, v * vec))
+                    L.append('      if (R.xs + %d <= (int)A.shape[2]) %s(q%d + %d, &o%d[%d]);'
+                             % ((v + 1) * vec, store, fi, v * vec, fi, v * vec))
             L.append('    }')
         L.append('  }')
         L.append('}')

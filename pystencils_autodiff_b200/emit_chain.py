@@ -43,6 +43,9 @@ __all__ = ['chain_ineligible_reason', 'emit_march_chain']
 
 
 def chain_ineligible_reason(ir: StencilKernelIR) -> Optional[str]:
+    if any(f.dtype.numpy_dtype == np.dtype(np.float16) for f in ir.all_fields):
+        # a pair would carry the intermediate field in fp32 and round once, two launches round it to fp16 in between
+        return 'float16 fields: fused pairs not implemented'
     reason = march_ineligible_reason(ir)
     if reason:
         return reason

@@ -4,6 +4,7 @@ contains the full-barrier wait of the consumer warps), and what that loop costs 
 
     python scripts/sass_stats.py c5            # forward + adjoint march kernels of a workload
     python scripts/sass_stats.py c3 x2         # the fused-pair kernel
+    python scripts/sass_stats.py c3 float16    # the workload with float16 fields
 For an issue-bound kernel (C5: sqrt / division chains) time ~ loop instructions x warp-steps / (SMs x 4 x clock)."""
 import collections
 import os
@@ -80,8 +81,9 @@ def report(ek, label, cells_per_step, cells):
 
 def main():
     name = sys.argv[1] if len(sys.argv) > 1 else 'c5'
-    x2 = len(sys.argv) > 2 and sys.argv[2] == 'x2'
-    op = make_config(name)
+    x2 = 'x2' in sys.argv[2:]
+    dtype = next((a for a in sys.argv[2:] if a.startswith('float')), None)
+    op = make_config(name, dtype=dtype)
     cells = 1
     for s_ in CONFIG_SHAPES[name]['shape']:
         cells *= s_
