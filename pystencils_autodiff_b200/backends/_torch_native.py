@@ -36,6 +36,11 @@ def numpy_dtype_to_torch(dtype):
     return getattr(torch, np.dtype(dtype).name)
 
 
+def launch_schedule(steps, pairs):
+    """Steps per launch for ``steps`` applications of a stencil: fused pairs and the odd last step, or single steps."""
+    return [2] * (steps // 2) + [1] * (steps % 2) if pairs else [1] * steps
+
+
 class CompiledKernel:
     """One lowered kernel, callable like the reference's ``call_<kernel>(**tensors, **scalars)`` wrapper
     (backends/astnodes.py:143-146): fields are passed by name, outputs are written in place."""
@@ -131,8 +136,7 @@ class CompiledKernel:
                                                                 'tensor layout needs the generic kernel'))
         # pairs wherever they can be built: every measured case wins (round 2, scripts/steps_bench.py: 7-point fp32 1024^3
         # 1.62x, 5-point fp32 8192^2 — lifted to a one-plane 3-D field — 1.39x, 27-point fp64 768^3 1.11x)
-        pair = can_pair if fuse is None else bool(fuse)
-        launches = [2] * (steps // 2) + [1] * (steps % 2) if pair else [1] * steps
+        launches = launch_schedule(steps, can_pair if fuse is None else fuse)
         out = torch.empty_like(src) if out is None else out
         if out.data_ptr() == src.data_ptr():
             raise ValueError('%s: run_steps cannot work in place (out is src)' % self.function_name)

@@ -26,7 +26,7 @@ from collections import OrderedDict
 import numpy as np
 
 from . import runtime
-from .backends._torch_native import CompiledKernel, numpy_dtype_to_torch
+from .backends._torch_native import CompiledKernel, launch_schedule, numpy_dtype_to_torch
 
 __all__ = ['SlabDecomposition', 'HaloExchanger', 'SlabDataHandling', 'GraphDataHandling', 'PyTorchDataHandling',
            'create_slab_autograd_function', 'create_slab_unrolled_function',
@@ -35,8 +35,6 @@ __all__ = ['SlabDecomposition', 'HaloExchanger', 'SlabDataHandling', 'GraphDataH
 
 import enum as _enum
 import os as _os
-_PEER_NEVER_WAIT = bool(_os.environ.get('PSAD_PEER_NEVER_WAIT'))    # timing experiments only: results are then unordered
-_ALWAYS_ORDER_SIDE_LAUNCHES = bool(_os.environ.get('PSAD_ALWAYS_ORDER_SIDE'))     # diagnostic switch (scripts/r2_ab_multi.sh)
 
 
 class SlabDecomposition:
@@ -148,6 +146,37 @@ def slab_ranges(global_shape, start, n, g, has_lo, has_hi, boundary, margin, ndi
     if lo_w == 0 and hi_w == 0:
         return rng(g, g + n), None, None
     return rng(g + lo_w, g + n - hi_w), (rng(g, g + lo_w) if lo_w else None), (rng(g + n - hi_w, g + n) if hi_w else None)
+
+
+def _reach(ir, name):
+    """How many planes along dim 0 (the decomposed axis) ``ir`` reads field ``name`` away from the centre."""
+    return max(ir.halo(name)[0])
+
+
+def _exchanged_inputs(ir, dec):
+    """Names of the input fields of ``ir`` whose ghost planes must be refreshed before a launch on ``dec``: ghost planes
+    come from a neighbouring rank or, on a periodic domain, possibly from this rank's own far side."""
+    if not (dec.world_size > 1 or dec.periodic) or dec.g == 0:
+        return []
+    return [f.name for f in ir.input_fields if _reach(ir, f.name) > 0]
+
+
+def _fused_pair_reason(kernel, dec):
+    """None when ``out = S(S(u))`` of ``kernel`` can run as one launch (``run_kernel(..., fused_steps=2)``) on ``dec``,
+    else why not.  It is also the default wherever pairs are optional: every measured case wins (3-D 7-point fp32 1024^3
+    per GPU: 1.63x / 1.71x at one / two GPUs; 27-point fp64 768^3: 1.08x / 1.07x, profiles/r2_slab_steps_c*_n*.json;
+    2-D 5-point fp32 8192^2: 1.39x)."""
+    ir = kernel.ir
+    why = kernel.fused_steps_reason()
+    if why is None and ir.ndim != 3:
+        if dec.world_size > 1 or dec.g > 0:
+            why = 'pairs of 2-D fields run on whole arrays only (one rank, no ghost planes)'
+    elif why is None and (dec.world_size > 1 or dec.periodic):       # (one periodic rank is its own neighbour)
+        need = 2 * _reach(ir, ir.input_fields[0].name)
+        if dec.g < need:
+            why = ('a pair needs %d ghost planes along dim 0 (twice the reach of the stencil), the data handling '
+                   'stores %d ghost layers' % (need, dec.g))
+    return None if why is None else '%s: steps cannot be fused: %s' % (kernel.function_name, why)
 
 
 class HaloExchanger:
@@ -346,14 +375,7 @@ class _PeerHalo:
             self.fence()
         key = (id(kernel), fused_steps)
         if key not in self._ranges:
-            halo = max(ir.halo(ir.input_fields[0].name)[0]) if fused_steps > 1 else None
-            if fused_steps > 1:
-                reason = kernel.fused_steps_reason()
-                if reason:
-                    raise ValueError('%s: steps cannot be fused: %s' % (kernel.function_name, reason))
-                if dec.g < fused_steps * halo:
-                    raise ValueError('%d fused steps of a stencil reaching %d plane(s) need %d ghost planes, the slab stores %d'
-                                     % (fused_steps, halo, fused_steps * halo, dec.g))
+            halo = _reach(ir, ir.input_fields[0].name) if fused_steps > 1 else None
             # ONE launch for all owned planes: nothing waits for an exchange
             whole = slab_ranges(dec.global_shape, dec.start, dec.n_local, dec.g, False, False, ir.boundary, ir.ghost_layers,
                                 ir.ndim, fused_steps, halo, periodic=dec.periodic)[0]
@@ -381,9 +403,7 @@ class _PeerHalo:
                 self.structs.clear()
             self.structs[skey] = peer
         self.seq += 1
-        peer.expect = 0 if _PEER_NEVER_WAIT else self.seq - 1
-        if fused_steps > 1:
-            kwargs = dict(kwargs, _variant='march_x2')
+        peer.expect = self.seq - 1
         kernel(**arrays, **kwargs, _range=whole, _peer=peer)
         runtime.stream_write_u32(self.flags.data_ptr(), self.seq, self.torch.cuda.current_stream(dh.device).cuda_stream)
 
@@ -735,16 +755,22 @@ class SlabDataHandling:
     def start_exchange(self, name):
         """Asynchronous: exchange on the communication stream, ordered after everything already queued on the
         current stream."""
-        if self.dec.g == 0 or name in self._replicated:
+        if name in self._replicated:
+            return False
+        return self._start_exchange(self.gpu_arrays[name])
+
+    def _start_exchange(self, t):
+        """``start_exchange`` of the slab array ``t``; True where the communication stream was ordered behind the current
+        one."""
+        if self.dec.g == 0:
             return False
         if self.dec.world_size == 1:
             if self.dec.periodic:
                 # one rank on a periodic domain is its own neighbour: two device copies on the current stream
-                t, g, n = self.gpu_arrays[name], self.dec.g, self.dec.n_local
+                g, n = self.dec.g, self.dec.n_local
                 t[:g].copy_(t[n:n + g])
                 t[n + g:].copy_(t[g:2 * g])
             return False
-        t = self.gpu_arrays[name]
         if t.is_cuda:
             comm = self._streams()
             cur = self.torch.cuda.current_stream(self.device)
@@ -795,58 +821,63 @@ class SlabDataHandling:
                             'the Function class of a torch_native op; arbitrary callables only on a single rank')
         if fused_steps not in (1, 2):
             raise ValueError('fused_steps must be 1 or 2')
+        arrays = {f.name: self.gpu_arrays[f.name] for f in kernel.fields}
+        replicated = [n for n in arrays if n in self._replicated]
+        if not replicated:
+            return self._launch(kernel, arrays, halo_fields, fused_steps, kwargs)
+        self._record_launch(kernel, halo_fields, fused_steps)
+        if len(replicated) != len(arrays):
+            raise ValueError('%s mixes slab-decomposed arrays with arrays of their own shape (%s)'
+                             % (kernel.function_name, ', '.join(sorted(replicated))))
+        if fused_steps > 1:
+            kwargs = dict(kwargs, _variant='march_x2')
+        return kernel(**arrays, **kwargs)          # whole arrays, every rank, no exchange
+
+    def _record_launch(self, kernel, halo_fields, fused_steps):
         for n in halo_fields:           # recorded in the reference's order: synchronisation, then the kernel call
             self._record(('Communication', n, None, True))
         self._record(('KernelCall', kernel.function_name) if fused_steps == 1 else
                      ('KernelCall', kernel.function_name, fused_steps))
-        arrays = {f.name: self.gpu_arrays[f.name] for f in kernel.fields}
         if kernel.function_name not in self.kernel_io:          # for computationgraph.ComputationGraph
             self.kernel_io[kernel.function_name] = ([f.name for f in kernel.ir.input_fields],
                                                     [f.name for f in kernel.ir.output_fields])
-        replicated = [n for n in arrays if n in self._replicated]
-        if replicated:
-            if len(replicated) != len(arrays):
-                raise ValueError('%s mixes slab-decomposed arrays with arrays of their own shape (%s)'
-                                 % (kernel.function_name, ', '.join(sorted(replicated))))
-            if fused_steps > 1:
-                kwargs = dict(kwargs, _variant='march_x2')
-            return kernel(**arrays, **kwargs)          # whole arrays, every rank, no exchange
-        ir = kernel.ir
-        if fused_steps > 1 and ir.ndim != 3 and self.dec.world_size == 1 and self.dec.g == 0:
-            # the arrays ARE the field (one rank, no ghost planes): the 2-D pair runs on them whole, like
-            # CompiledKernel.run_steps (lifted to a one-plane 3-D field by the emitter)
-            reason = kernel.fused_steps_reason()
-            if reason:
-                raise ValueError('%s: steps cannot be fused: %s' % (kernel.function_name, reason))
-            return kernel(**arrays, **dict(kwargs, _variant='march_x2'))
-        if self.peer is not None and self.peer.applies(kernel, arrays, fused_steps):
-            return self.peer.run(kernel, arrays, fused_steps, kwargs)
+
+    def _launch(self, kernel, arrays, halo_fields, fused_steps, kwargs):
+        """``run_kernel`` on the given slab arrays (field name -> tensor with ghost planes) instead of the registered
+        ones."""
+        self._record_launch(kernel, halo_fields, fused_steps)
         key = (id(kernel), fused_steps)
         if key not in self._range_cache:
-            if fused_steps > 1:
-                reason = kernel.fused_steps_reason()
-                if reason:
-                    raise ValueError('%s: steps cannot be fused: %s' % (kernel.function_name, reason))
-                if ir.ndim != 3:
-                    raise ValueError('%s: fused steps on slabs need 3-D fields' % kernel.function_name)
-                halo = max(ir.halo(ir.input_fields[0].name)[0])
-                ranges = self.dec.ranges(ir.boundary, ir.ghost_layers, ir.ndim, fused_steps, halo)
-            else:
+            ir = kernel.ir
+            if fused_steps == 1:
                 ranges = self.dec.ranges(ir.boundary, ir.ghost_layers, ir.ndim)
+            else:
+                reason = _fused_pair_reason(kernel, self.dec)
+                if reason:
+                    raise ValueError(reason)
+                # None for 2-D pairs: the arrays ARE the field (one rank, no ghost planes), the pair runs on them whole
+                # like CompiledKernel.run_steps (lifted to a one-plane 3-D field by the emitter)
+                ranges = None if ir.ndim != 3 else self.dec.ranges(ir.boundary, ir.ghost_layers, ir.ndim, fused_steps,
+                                                                   _reach(ir, ir.input_fields[0].name))
             self._range_cache[key] = (kernel, ranges)      # holds the kernel: its id() cannot be reused while cached
-        interior, lo, hi = self._range_cache[key][1]
+        ranges = self._range_cache[key][1]
         if fused_steps > 1:
             kwargs = dict(kwargs, _variant='march_x2')
+        if ranges is None:
+            return kernel(**arrays, **kwargs)
+        if self.peer is not None and self.peer.applies(kernel, arrays, fused_steps):
+            return self.peer.run(kernel, arrays, fused_steps, kwargs)
+        interior, lo, hi = ranges
         if self.peer is not None:
             self.peer.before_foreign_launch()     # the neighbours may still be reading what this launch overwrites
-        ordered = [self.start_exchange(n) for n in halo_fields]      # True where the comm stream was ordered behind `cur`
+        ordered = [self._start_exchange(arrays[n]) for n in halo_fields]     # True where the comm stream waits for `cur`
         side = [r for r in (lo, hi) if r is not None]
         on_comm = bool(side) and self._comm_stream is not None and all(t.is_cuda for t in arrays.values())
         if on_comm:
             # the side launches read inputs produced on the current stream (and write outputs whose previous user may
             # still be pending there): order the communication stream behind it even when no exchange was started
             # in this call (start_exchange records the same dependency; a second record / wait is harmless)
-            if not any(ordered) or _ALWAYS_ORDER_SIDE_LAUNCHES:
+            if not any(ordered):
                 self._ev_ready.record(self.torch.cuda.current_stream(self.device))
                 self._comm_stream.wait_event(self._ev_ready)
             for r in side:
@@ -872,39 +903,21 @@ class SlabDataHandling:
         ``fuse=True``: pairs of steps run as one launch with one exchange of ``2 * halo`` ghost planes
         (``run_kernel(..., fused_steps=2)``): per pair the field is read and written once instead of twice and one
         message per neighbour replaces two.  Needs ``default_ghost_layers >= 2 * halo``.  Default (``fuse=None``): pairs
-        wherever they are a measured win and possible — 3-D fields (7-point fp32, 1024^3 per GPU:
-        1.63x at one GPU, 1.71x at two, profiles/r2_slab_steps_c3_n*.json) on a data handling that stores enough ghost
-        layers, 8-byte elements too (27-point fp64 768^3: 1.08x at one GPU, 1.07x at two, profiles/r2_slab_steps_c4_n*.json),
-        2-D 'zeros' stencils on one rank without ghost planes; everything else runs single steps (``_pairs_pay_off``)."""
+        wherever they can run (``_fused_pair_reason``): 3-D fields on a data handling that stores enough ghost layers,
+        2-D 'zeros' stencils on one rank without ghost planes; everything else runs single steps."""
         ir = kernel.ir
         if len(ir.input_fields) != 1 or len(ir.output_fields) != 1:
             raise ValueError('%s: run_steps needs a kernel with one input and one output field' % kernel.function_name)
         if steps < 0:
             raise ValueError('steps must be >= 0')
         fin, fout = ir.input_fields[0].name, ir.output_fields[0].name
-        # ghost planes come from a neighbouring rank — or, on a periodic domain, possibly from this rank's own far side
-        halo = [fin] if (self.dec.world_size > 1 or self.dec.periodic) and self.dec.g > 0 and max(ir.halo(fin)[0]) > 0 else []
+        halo = _exchanged_inputs(ir, self.dec)
         if fuse is None:
-            fuse = _pairs_pay_off(kernel, self.dec)
-        launches = [2] * (steps // 2) + [1] * (steps % 2) if fuse else [1] * steps
-        for n in launches:
+            fuse = _fused_pair_reason(kernel, self.dec) is None
+        for n in launch_schedule(steps, fuse):
             self.run_kernel(kernel, halo_fields=halo, fused_steps=n, **scalars)
             self.swap(fin, fout)
         return self.gpu_arrays[fin]
-
-
-def _pairs_pay_off(kernel, dec):
-    """Default of ``fuse=None``: fused pairs of steps wherever they can run — every measured case wins: 3-D fields on any
-    number of ranks when the slab stores the ``2 x reach`` ghost planes a pair needs (7-point fp32 1024^3 per GPU: 1.63x /
-    1.71x at one / two GPUs; 27-point fp64 768^3: 1.08x / 1.07x, profiles/r2_slab_steps_c4_n*.json), 2-D 'zeros' stencils on
-    one rank without ghost planes (5-point fp32 8192^2: 1.4x)."""
-    ir = kernel.ir
-    if kernel.fused_steps_reason() is not None:
-        return False
-    if ir.ndim != 3:      # 2-D pairs (5-point fp32 8192^2: 1.39x) run on whole arrays only: one rank, no ghost planes
-        return ir.ndim == 2 and dec.world_size == 1 and dec.g == 0
-    reach = max(ir.halo(ir.input_fields[0].name)[0])
-    return (dec.world_size == 1 and not dec.periodic) or dec.g >= 2 * reach
 
 
 class _SlabTensors:
@@ -948,19 +961,8 @@ class _SlabTensors:
         return padded[self.g:self.g + self.n]
 
     def launch(self, kernel, arrays, halo, scalars, fused_steps=1):
-        dh = self.dh
-        arrays = {k: v for k, v in arrays.items() if k in {f.name for f in kernel.fields}}
-        keep = {k: dh.gpu_arrays.get(k) for k in arrays}
-        dh.gpu_arrays.update(arrays)                 # run_kernel looks its fields up by name at call time
-        try:
-            dh.run_kernel(kernel, halo_fields=[h for h in halo if h in arrays], fused_steps=fused_steps,
-                          **{k: v for k, v in scalars.items() if k in kernel.scalars})
-        finally:
-            for k, v in keep.items():
-                if v is None:
-                    dh.gpu_arrays.pop(k, None)
-                else:
-                    dh.gpu_arrays[k] = v
+        self.dh._launch(kernel, {f.name: arrays[f.name] for f in kernel.fields}, halo, fused_steps,
+                        {k: v for k, v in scalars.items() if k in kernel.scalars})
 
 
 def _slab_tensors(data_handling):
@@ -973,7 +975,7 @@ def _check_scalars(kernels, scalars):
     for kern in kernels:
         missing = [s_ for s_ in kern.scalars if s_ not in scalars]
         if missing:
-            raise TypeError('%s: missing scalar argument(s) %s (pass scalars={...})' % (kern.function_name, missing))
+            raise TypeError('%s: missing scalar argument(s) %s' % (kern.function_name, missing))
 
 
 def create_slab_autograd_function(op, data_handling, op_name=None, tuning=None, scalars=None, kernel_class=None):
@@ -1014,14 +1016,12 @@ def create_slab_autograd_function(op, data_handling, op_name=None, tuning=None, 
         if fwd is not None:
             (grad_of if fwd in fwd_outputs else adjoint_of)[fwd.name] = f.name
     sharded = dec.world_size > 1 or dec.periodic       # ghost planes are filled from a neighbour (possibly this rank)
-
-    def reach(ir, name):
-        return max(ir.halo(name)[0])
-    need = max([reach(ir, f.name) for ir in (fwd_ir, bwd_ir) for f in ir.input_fields] + [0])
+    need = max([_reach(ir, f.name) for ir in (fwd_ir, bwd_ir) for f in ir.input_fields] + [0])
     if sharded and g < need:
         raise ValueError('the stencils reach %d plane(s) along dim 0, the data handling stores %d ghost layer(s)' % (need, g))
-    fwd_halo = [f.name for f in fwd_ir.input_fields if sharded and reach(fwd_ir, f.name) > 0]
-    bwd_halo = [f.name for f in bwd_ir.input_fields if sharded and reach(bwd_ir, f.name) > 0 and f.name not in fwd_halo]
+    fwd_halo = _exchanged_inputs(fwd_ir, dec)
+    # the forward pass has refreshed the ghost planes of its inputs, and the backward pass reuses those buffers
+    bwd_halo = [n for n in _exchanged_inputs(bwd_ir, dec) if n not in fwd_halo]
     fwd_reads = {f.name for f in fwd_ir.input_fields}
     bwd_reads = {f.name for f in bwd_ir.input_fields}
 
@@ -1106,24 +1106,24 @@ def create_slab_unrolled_function(op, data_handling, steps, fuse=None, op_name=N
     scalars = dict(scalars or {})
     _check_scalars((fwd_k, bwd_k), scalars)
     sharded = dec.world_size > 1 or dec.periodic       # ghost planes are filled from a neighbour (possibly this rank)
-    if fuse is None:
-        fuse = _pairs_pay_off(fwd_k, dec) and _pairs_pay_off(bwd_k, dec)
-    launches = [2] * (steps // 2) + [1] * (steps % 2) if fuse else [1] * steps
+    reason = _fused_pair_reason(fwd_k, dec) or _fused_pair_reason(bwd_k, dec)
+    if fuse and reason:
+        raise ValueError(reason)
+    launches = launch_schedule(steps, reason is None if fuse is None else fuse)
     for kern in (fwd_k, bwd_k):
         ir = kern.ir
-        reach = max(ir.halo(ir.input_fields[0].name)[0])
-        if fuse and kern.fused_steps_reason():
-            raise ValueError('%s: steps cannot be fused: %s' % (kern.function_name, kern.fused_steps_reason()))
-        if sharded and dec.g < reach * max(launches):
-            raise ValueError('%s reaches %d plane(s) per step: %d fused step(s) need %d ghost layers, the data handling '
-                             'stores %d' % (kern.function_name, reach, max(launches), reach * max(launches), dec.g))
+        reach = _reach(ir, ir.input_fields[0].name)
+        if sharded and dec.g < reach:
+            raise ValueError('%s reaches %d plane(s) along dim 0, the data handling stores %d ghost layers'
+                             % (kern.function_name, reach, dec.g))
+    halos = {k: _exchanged_inputs(k.ir, dec) for k in (fwd_k, bwd_k)}
 
     def run(kernel, t):
         ir = kernel.ir
         fin, fout = ir.input_fields[0], ir.output_fields[0]
         dtype = numpy_dtype_to_torch(fin.dtype.numpy_dtype)
         cur = pool.padded_of(t if t.is_contiguous() else t.contiguous(), dtype, '%s: field %r' % (op.op_name, fin.name))
-        halo = [fin.name] if sharded and max(ir.halo(fin.name)[0]) > 0 else []
+        halo = halos[kernel]
         spare = [pool.new_padded(dtype, t, zero=False) for _ in range(min(2, len(launches)))]
         for i, k in enumerate(launches):
             dst = spare[i % len(spare)]
@@ -1280,8 +1280,8 @@ class TimeLoop:
 
         The reference's time-loop idiom — ``add_call(kernel)`` then ``swap(in, out)`` (graph_datahandling.py:152-197, the
         pair ``merge_swaps_with_kernel_calls`` folds into one node, :329-344) — is recognised when the kernel is a
-        one-field stencil whose pair the emitter can build (``CompiledKernel.fused_steps_reason``) and, for the default
-        ``fuse_steps=None``, where ``SlabDataHandling.run_steps`` fuses by default (``_pairs_pay_off``).  ``run`` then
+        one-field stencil whose pair can run on this data handling (``_fused_pair_reason``, the rule
+        ``SlabDataHandling.run_steps`` fuses by), for the default ``fuse_steps=None`` and ``True`` alike.  ``run`` then
         issues ``out = S(S(u))`` + one swap per two time steps — one read and one write of the field, one halo exchange of
         twice the reach — exactly what ``run_steps`` does, through the reference's API.  Results can differ from single
         steps in the last bit (sums are ordered differently)."""
@@ -1309,21 +1309,13 @@ class TimeLoop:
                 all(isinstance(v, (int, float)) and not isinstance(v, bool) for v in kw.values())
             why = 'the swap does not exchange the kernel\'s input and output arrays (or the call passes non-scalar arguments)'
         if ok:
-            reason = kernel.fused_steps_reason()
-            ok, why = reason is None, reason
-        if ok and self.fuse_steps is None:
-            ok = _pairs_pay_off(kernel, self.dh.dec)
-        elif ok:
-            reach = max(ir.halo(fin)[0])
-            ok = (self.dh.dec.world_size == 1 and not self.dh.dec.periodic) or self.dh.dec.g >= 2 * reach
-            why = 'a fused pair needs %d ghost layers along dim 0, the data handling stores %d' % (2 * reach, self.dh.dec.g)
+            why = _fused_pair_reason(kernel, self.dh.dec)
+            ok = why is None
         if not ok:
             if self.fuse_steps is True:
                 raise ValueError('TimeLoop(fuse_steps=True): %s' % why)
             return None
-        dec = self.dh.dec
-        needs_halo = (dec.world_size > 1 or dec.periodic) and dec.g > 0 and max(ir.halo(fin)[0]) > 0
-        return kernel, dict(kw), ((fin,) if needs_halo else ())
+        return kernel, dict(kw), tuple(_exchanged_inputs(ir, self.dh.dec))
 
     def _one_pair(self, fused):
         kernel, kw, halo = fused
@@ -1493,13 +1485,9 @@ class SlabStencilOp:
             names.setdefault(f.name, f)
         for n, f in names.items():
             self.dh.add_array(n, dtype=f.dtype.numpy_dtype)
-        fwd_ir, bwd_ir = op.forward_ast_gpu, op.backward_ast_gpu
-        self.fwd_halo = [f.name for f in fwd_ir.input_fields if max(fwd_ir.halo(f.name)[0]) > 0] if g else []
-        self.bwd_halo = [f.name for f in bwd_ir.input_fields if max(bwd_ir.halo(f.name)[0]) > 0] if g else []
-        for kern in (self.fwd, self.bwd):
-            missing = [s_ for s_ in kern.scalars if s_ not in scalars]
-            if missing:
-                raise TypeError('%s: missing scalar argument(s) %s (pass scalars={...})' % (kern.function_name, missing))
+        self.fwd_halo = _exchanged_inputs(op.forward_ast_gpu, self.dh.dec)
+        self.bwd_halo = _exchanged_inputs(op.backward_ast_gpu, self.dh.dec)
+        _check_scalars((self.fwd, self.bwd), scalars)
         self.scalars = scalars
         self.fwd_scalars = {s_: scalars[s_] for s_ in self.fwd.scalars}
         self.bwd_scalars = {s_: scalars[s_] for s_ in self.bwd.scalars}
@@ -1696,10 +1684,7 @@ class HostStreamedOp:
         ``host_out``: name -> pinned CPU tensor receiving every output (forward outputs and ``diff<in>``);
         ``scalars``: values of the free scalar symbols of the kernels."""
         torch = self.torch
-        for kern in (self.fwd, self.bwd):
-            missing = [s_ for s_ in kern.scalars if s_ not in scalars]
-            if missing:
-                raise TypeError('%s: missing scalar argument(s) %s' % (kern.function_name, missing))
+        _check_scalars((self.fwd, self.bwd), scalars)
         g, C, N0 = self.g, self.chunk, self.shape[0]
         cur = torch.cuda.current_stream(self.device)
         start = torch.cuda.Event()

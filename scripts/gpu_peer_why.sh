@@ -7,5 +7,4 @@ run() {  # tag, env, args
   timeout 420 env $2 $TR --master-port 2954$((RANDOM % 10)) scripts/check_peer_halo.py $3 > gpurun_out/r2_peerwhy_$1.log 2>&1
   echo "== $1 ($2 $3) rc=$?"; grep "^{\|Error" gpurun_out/r2_peerwhy_$1.log | tail -3
 }
-run c4_768_nowait "PSAD_CHECK_SHAPE=768,768,768 PSAD_PEER_NEVER_WAIT=1" "c4 zeros 3 --time"
 run c4_768_memset "PSAD_CHECK_SHAPE=768,768,768 PSAD_PEER_STREAM_SIGNAL=1" "c4 zeros 3 --time"

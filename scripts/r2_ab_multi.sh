@@ -5,7 +5,7 @@ mkdir -p gpurun_out
 R="python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1"
 B="bench.py --gpus $N --steps 20 --warmup 5 --no-e2e"
 i=0
-for arm in "" "PSAD_BENCH_NO_NVML=1" "PSAD_ALWAYS_ORDER_SIDE=1" "PSAD_NO_LAUNCH_CACHE=1" "" "PSAD_BENCH_NO_NVML=1"; do
+for arm in "" "PSAD_BENCH_NO_NVML=1" "PSAD_NO_LAUNCH_CACHE=1" "" "PSAD_BENCH_NO_NVML=1"; do
   i=$((i+1))
   env $arm $R --master-port $((29530+i)) $B > gpurun_out/r2_ab_n${N}_$i.json 2> gpurun_out/r2_ab_n${N}_$i.err
   python - "$arm" gpurun_out/r2_ab_n${N}_$i.json <<'PY'
