@@ -23,6 +23,7 @@ import numpy as np
 
 from ..emit import emit_generic, emit_march, march_ineligible_reason
 from ..emit_chain import chain_ineligible_reason, emit_march_chain
+from ..field import BFLOAT16, BasicType
 from ..ir import StencilKernelIR, lift_to_3d, split_index_components
 from .. import runtime
 
@@ -31,9 +32,10 @@ __all__ = ['create_autograd_function', 'create_unrolled_function', 'compile_kern
 
 
 def numpy_dtype_to_torch(dtype):
-    """dtype name mapping (reference: backends/_pytorch.py:95-97)."""
+    """dtype name mapping (reference: backends/_pytorch.py:95-97); ``'bfloat16'`` / ``BFLOAT16`` -> ``torch.bfloat16``."""
     import torch
-    return getattr(torch, np.dtype(dtype).name)
+    dt = BasicType(dtype).numpy_dtype
+    return torch.bfloat16 if dt == BFLOAT16 else getattr(torch, dt.name)
 
 
 def launch_schedule(steps, pairs):

@@ -13,7 +13,7 @@ from .field import fields
 
 __all__ = ['readme_op', 'diffusion2d_op', 'heat3d_op', 'stencil27_op', 'tv_gradient_op', 'CONFIG_SHAPES', 'make_config']
 
-_DT = {'float16': 'float16', 'float32': 'float32', 'float64': 'float64'}
+_DT = {'bfloat16': 'bfloat16', 'float16': 'float16', 'float32': 'float32', 'float64': 'float64'}
 
 
 def _shape_str(shape):

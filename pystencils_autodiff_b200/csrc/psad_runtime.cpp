@@ -645,6 +645,8 @@ static int encode_one_map(const psad_plan_t& P, const psad_field_plan_t& fp, voi
   unsigned estr[3] = {1, 1, 1};
   for (int d = 0; d < nd; ++d)
     if (box[d] < 1 || box[d] > 256) return fail(PSAD_ERR_INVALID, "TMA box dim %d = %u out of range", d, box[d]);
+  // Every 2-byte field, bfloat16 included, is encoded as FLOAT16: a tiled load with zero out-of-bounds fill copies bits
+  // unchanged, and the fill word 0x0000 is +0 in both formats.
   const int dtype = fp.elem_size == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16
                     : fp.elem_size == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT64;
   CUresult r = g_drv.cuTensorMapEncodeTiled(out, dtype,

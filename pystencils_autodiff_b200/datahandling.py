@@ -27,6 +27,7 @@ import numpy as np
 
 from . import runtime
 from .backends._torch_native import CompiledKernel, launch_schedule, numpy_dtype_to_torch
+from .field import BFLOAT16, BasicType, numpy_dtype_of_torch
 
 __all__ = ['SlabDecomposition', 'HaloExchanger', 'SlabDataHandling', 'GraphDataHandling', 'PyTorchDataHandling',
            'create_slab_autograd_function', 'create_slab_unrolled_function',
@@ -35,6 +36,12 @@ __all__ = ['SlabDecomposition', 'HaloExchanger', 'SlabDataHandling', 'GraphDataH
 
 import enum as _enum
 import os as _os
+
+
+def _host_array(t):
+    """numpy copy of a tensor; bfloat16 is widened to float32 (exactly), numpy has no bfloat16."""
+    import torch
+    return (t.float() if t.dtype == torch.bfloat16 else t).cpu().numpy()
 
 
 class SlabDecomposition:
@@ -530,7 +537,7 @@ class SlabDataHandling:
         self._ev_halo = None
         # peer halos: the stencil kernels read their ghost planes from the neighbouring GPUs' arrays (CUDA IPC mappings,
         # NVLink) instead of having them exchanged first — see _PeerHalo
-        # float16 arrays always take the NCCL exchange: the peer-halo kernel instance is not built for them
+        # float16 and bfloat16 arrays always take the NCCL exchange: the peer-halo kernel instance is not built for them
         self._peer_forced = peer_halo is True
         if peer_halo == 'auto':
             peer_halo = peer_halos_pay_off(self.dec.local_shape, self.dec.world_size, backend, self.device)
@@ -573,11 +580,12 @@ class SlabDataHandling:
             self._replicated.add(name)
         else:
             shape = self.dec.local_shape
+        dtype = BasicType(dtype).numpy_dtype
         arr = self.torch.zeros(shape + tail, dtype=numpy_dtype_to_torch(dtype), device=self.device)
-        if self.peer is not None and np.dtype(dtype) == np.float16 and name not in self._replicated:
+        if self.peer is not None and dtype in (np.float16, BFLOAT16) and name not in self._replicated:
             if self._peer_forced:
-                raise ValueError('peer halos are not available for float16 arrays (peer_halo=False or \'auto\' exchange '
-                                 'their ghost planes through NCCL)')
+                raise ValueError('peer halos are not available for %s arrays (peer_halo=False or \'auto\' exchange '
+                                 'their ghost planes through NCCL)' % ('bfloat16' if dtype == BFLOAT16 else 'float16'))
             # 'auto': not registered, so every launch on this array takes the NCCL exchange (_PeerHalo.applies)
         elif self.peer is not None and name not in self._replicated:
             self.peer.register(arr)              # collective: every rank adds its arrays in the same order
@@ -614,7 +622,7 @@ class SlabDataHandling:
 
     def add_array_like(self, name, name_of_template_field):
         t = self.gpu_arrays[name_of_template_field]
-        return self.add_array(name, dtype=np.dtype(str(t.dtype).replace('torch.', '')))
+        return self.add_array(name, dtype=numpy_dtype_of_torch(t.dtype))
 
     def fill(self, array_name, val, **_):
         self._record(('Fill', array_name))        # graph_datahandling.py:324-327 records 'Fill <name>'
@@ -642,13 +650,14 @@ class SlabDataHandling:
 
     def save_fields(self, fields, output_path, flag_field=None):
         """Records a ``FieldOutput`` marker like the reference (graph_datahandling.py:346-350) and writes this rank's
-        owned planes to ``<output_path>.rank<r>.npz``."""
+        owned planes to ``<output_path>.rank<r>.npz``.  bfloat16 arrays are written as float32 (an exact widening:
+        numpy has no bfloat16)."""
         if isinstance(fields, str) or not hasattr(fields, '__iter__'):
             fields = [fields]
         names = [f if isinstance(f, str) else f.name for f in fields]
         self._record(('FieldOutput', tuple(names), output_path, flag_field))
         np.savez('%s.rank%d.npz' % (output_path, self.dec.rank),
-                 **{n: self.owned(n).detach().cpu().numpy() for n in names})
+                 **{n: _host_array(self.owned(n).detach()) for n in names})
 
     def merge_swaps_with_kernel_calls(self, call_queue=None):
         """A ``Swap`` recorded right after a ``KernelCall`` is folded into that call
@@ -714,15 +723,16 @@ class SlabDataHandling:
         self.gpu_arrays[name1], self.gpu_arrays[name2] = self.gpu_arrays[name2], self.gpu_arrays[name1]
 
     def gather_array(self, name):
-        """Global array on every rank (host numpy), ghost planes stripped."""
+        """Global array on every rank (host numpy), ghost planes stripped.  A bfloat16 array is returned as float32 (an
+        exact widening: numpy has no bfloat16)."""
         import torch.distributed as dist
         local = self.owned(name).contiguous()
         if self.dec.world_size == 1 or name in self._replicated:
-            return local.cpu().numpy()
+            return _host_array(local)
         parts = [self.torch.empty((c,) + tuple(local.shape[1:]), dtype=local.dtype, device=local.device)
                  for c in self.dec.counts]
         dist.all_gather(parts, local) if len(set(self.dec.counts)) == 1 else self._all_gather_uneven(parts, local)
-        return self.torch.cat(parts, 0).cpu().numpy()
+        return _host_array(self.torch.cat(parts, 0))
 
     def _all_gather_uneven(self, parts, local):
         import torch.distributed as dist

@@ -23,16 +23,18 @@ import sympy as sp
 from sympy.codegen.ast import float32, float64, real
 from sympy.printing.c import C99CodePrinter
 
-from .field import Field
+from .field import BFLOAT16, Field
 from .ir import StencilKernelIR
 from .linopt import plan_linear
 
 KERNEL_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'csrc', 'kernels')
 EMITTER_VERSION = '19'
 
-_CT = {np.dtype(np.float16): 'psad_half', np.dtype(np.float32): 'float', np.dtype(np.float64): 'double'}
+_CT = {np.dtype(np.float16): 'psad_half', BFLOAT16: 'psad_bf16', np.dtype(np.float32): 'float',
+       np.dtype(np.float64): 'double'}
 _F16 = np.dtype(np.float16)
-# float16 fields: storage type psad_half (psad_half.cuh), values converted to fp32 where they enter the registers
+# 16-bit fields (float16, bfloat16): storage types psad_half / psad_bf16 (psad_half.cuh), values converted to fp32 where
+# they enter the registers
 HALF_HEADER = 'psad_half.cuh'
 # headers that only some kernels include: hashed into the cache key of those kernels only
 _OPTIONAL_HEADERS = (HALF_HEADER,)
@@ -247,7 +249,7 @@ def emit_generic(ir: StencilKernelIR, threads=256) -> EmittedKernel:
 
     L = _header(ir, 'generic')
     L += ['#include "psad_common.cuh"']
-    if any(f.dtype.numpy_dtype == _F16 for f in fields):
+    if any(f.dtype.itemsize == 2 for f in fields):
         L.append('#include "%s"' % HALF_HEADER)
     L += ['', 'typedef %s CT;' % CT]
     for f in fields:
@@ -373,8 +375,10 @@ def march_ineligible_reason(ir: StencilKernelIR) -> Optional[str]:
     for f in ir.all_fields:
         if f.index_dimensions:
             return 'index dimensions'
-        if f.dtype.numpy_dtype not in (_F16, np.dtype(np.float32), np.dtype(np.float64)):
+        if f.dtype.numpy_dtype not in (_F16, BFLOAT16, np.dtype(np.float32), np.dtype(np.float64)):
             return 'only float16/float32/float64 fields'
+    if len({f.dtype.numpy_dtype for f in ir.all_fields}) > 1 and any(f.dtype.numpy_dtype == BFLOAT16 for f in ir.all_fields):
+        return 'bfloat16 fields mixed with other field types'
     if len({f.dtype.numpy_dtype for f in ir.all_fields}) > 1 and any(f.dtype.numpy_dtype == _F16 for f in ir.all_fields):
         return 'float16 fields mixed with wider fields'
     if not ir.input_fields:
@@ -432,19 +436,20 @@ def _emit_march(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, maske
     scalars = [s.name for s in ir.scalars]
     nd = ir.ndim
     max_esize = max(f.dtype.itemsize for f in fields)
-    half = max_esize == 2     # all fields float16 (march_ineligible_reason): 8-byte vectors of 4 halves, fp32 window
+    half = max_esize == 2     # all fields float16 or all bfloat16 (march_ineligible_reason): 8-byte vectors of 4 cells,
+    #                           fp32 window
 
     def vec_cells(es):       # cells per shared load / global store vector
         return 4 if es == 2 else 16 // es
 
-    def reg_type(f):         # type of an output field's results in registers (rounded to fp16 only by the store)
+    def reg_type(f):         # type of an output field's results in registers (rounded to 16 bits only by the store)
         return CT if f.dtype.itemsize == 2 else _CT[f.dtype.numpy_dtype]
 
     # ---- geometry ------------------------------------------------------------------------------------------
     SX = t.sx or 4   # cells per thread along x: one 16-byte vector for 4-byte types, two for 8-byte types, one 8-byte
-    #                  vector for float16 (8 halves per lane would make the box 256 + pads wide: over the TMA limit)
+    #                  vector for 16-bit fields (8 cells per lane would make the box 256 + pads wide: over the TMA limit)
     if half and SX % 4:
-        raise ValueError('sx must be a multiple of 4 for float16 fields')
+        raise ValueError('sx must be a multiple of 4 for 16-bit fields')
     if not half and (SX * min(f.dtype.itemsize for f in fields)) % 16:
         raise ValueError('sx*itemsize must be a multiple of 16 bytes')
     TX = 32 * SX
@@ -459,7 +464,7 @@ def _emit_march(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, maske
         RY = t.ry or (2 if nd == 3 else 1)
         # cross-cell CSE keeps the shared temporaries of all the thread's cells live: 15+1 warps (128 registers) instead
         # of 16+1 (96) — TV-gradient adjoint 0.758 -> 0.722 ms, and 1.00 ms when it has to spill
-        # float16: the conversions take the 15+1-warp CSE tile over 128 registers (36 bytes spilled); 11+1 warps fit
+        # 16-bit fields: the conversions take the 15+1-warp CSE tile over 128 registers (36 bytes spilled); 11+1 warps fit
         TY = t.ty or (((22 if half else 30) if cross_cse else 32) if nd == 3 else 16)
     else:
         # 7 consumer warps + the producer warp = 8 warps: ptxas budgets registers for the CTA size rounded up to 4
@@ -492,7 +497,7 @@ def _emit_march(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, maske
         nbytes = boxw * boxh * es
         geo[f.name] = dict(ti=ti, es=es, vec=vec, nv=SX // vec, hz=h3[0], hy=h3[1], hx=h3[2], padl=padl, boxw=boxw,
                            boxh=boxh, bytes=nbytes, off=off, T=_CT[f.dtype.numpy_dtype],
-                           Tw='float' if es == 2 else _CT[f.dtype.numpy_dtype], ww=max(1, es // 4))   # window: fp16 as float
+                           Tw='float' if es == 2 else _CT[f.dtype.numpy_dtype], ww=max(1, es // 4))   # window: 16-bit as float
         off += -(-nbytes // 128) * 128
     STAGE_BYTES = off
     # ---- plane partial sums --------------------------------------------------------------------------------------

@@ -35,7 +35,7 @@ import sympy as sp
 
 from pystencils_autodiff_b200.emit import (FAST_MATH_OPTIONS, EmittedKernel, MarchTuning, _c_ident, _CT,
                                            _CudaPrinter, _header, _kernel_name, _off3, march_ineligible_reason)
-from pystencils_autodiff_b200.field import Field
+from pystencils_autodiff_b200.field import BFLOAT16, Field
 from pystencils_autodiff_b200.ir import StencilKernelIR
 from pystencils_autodiff_b200.linopt import plan_linear
 
@@ -46,6 +46,8 @@ def chain_ineligible_reason(ir: StencilKernelIR) -> Optional[str]:
     if any(f.dtype.numpy_dtype == np.dtype(np.float16) for f in ir.all_fields):
         # a pair would carry the intermediate field in fp32 and round once, two launches round it to fp16 in between
         return 'float16 fields: fused pairs not implemented'
+    if any(f.dtype.numpy_dtype == BFLOAT16 for f in ir.all_fields):
+        return 'bfloat16 fields: fused pairs not implemented'
     reason = march_ineligible_reason(ir)
     if reason:
         return reason

@@ -19,11 +19,15 @@ import numpy as np
 import sympy as sp
 
 __all__ = ['Field', 'FieldType', 'BasicType', 'fields', 'coerce_access', 'coerce_field',
-           'offset_to_direction_string', 'x_vector']
+           'offset_to_direction_string', 'x_vector', 'BFLOAT16']
+
+# numpy has no bfloat16: bfloat16 fields carry this 2-byte stand-in as their numpy dtype.  Their values only ever live in
+# torch.bfloat16 tensors; host copies (gather_array, save_fields) are widened to float32.
+BFLOAT16 = np.dtype([('bfloat16', '<u2')])
 
 _C_TYPE_NAMES = {
     'double': np.float64, 'float': np.float32, 'float64': np.float64, 'float32': np.float32,
-    'int': np.int32, 'int32': np.int32, 'int64': np.int64, 'float16': np.float16,
+    'int': np.int32, 'int32': np.int32, 'int64': np.int64, 'float16': np.float16, 'bfloat16': BFLOAT16,
 }
 
 
@@ -50,7 +54,7 @@ class BasicType:
     def c_name(self):
         return {np.dtype(np.float64): 'double', np.dtype(np.float32): 'float',
                 np.dtype(np.int32): 'int', np.dtype(np.int64): 'int64_t',
-                np.dtype(np.float16): 'half'}[self.numpy_dtype]
+                np.dtype(np.float16): 'half', BFLOAT16: 'bfloat16'}[self.numpy_dtype]
 
     @property
     def itemsize(self):
@@ -347,8 +351,13 @@ def _array_dtype(array):
     dt = array.dtype
     if isinstance(dt, np.dtype):
         return dt
-    # torch dtype
-    return np.dtype(str(dt).replace('torch.', ''))
+    return numpy_dtype_of_torch(dt)
+
+
+def numpy_dtype_of_torch(dtype):
+    """numpy dtype of a torch dtype: ``torch.bfloat16`` -> ``BFLOAT16``, the others by name."""
+    name = str(dtype).replace('torch.', '')
+    return BFLOAT16 if name == 'bfloat16' else np.dtype(name)
 
 
 # ---------------------------------------------------------------------------------------------

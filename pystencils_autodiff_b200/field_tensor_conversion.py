@@ -60,9 +60,10 @@ def coerce_to_field(field_name, array_like):
 def torch_tensor_from_field(field, init_val=0, cuda=True, requires_grad=False):
     """Tensor with the field's fixed shape and dtype (reference :132-137); CUDA by default."""
     import torch
+    from .backends._torch_native import numpy_dtype_to_torch
     if not field.has_fixed_shape:
         raise ValueError('field %s has no fixed shape' % field.name)
-    dtype = getattr(torch, field.dtype.numpy_dtype.name)
+    dtype = numpy_dtype_to_torch(field.dtype.numpy_dtype)
     shape = tuple(int(s) for s in field.shape)
     dev = 'cuda' if cuda else 'cpu'
     if init_val in (0, 0.0, False, None):

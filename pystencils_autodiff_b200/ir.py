@@ -19,7 +19,7 @@ import numpy as np
 import sympy as sp
 
 from .assignment import AssignmentCollection, coerce_assignments
-from .field import Field
+from .field import BFLOAT16, Field
 from .transformations import ConditionalFieldAccess
 
 __all__ = ['StencilKernelIR', 'KernelParameter', 'lower_assignments', 'split_index_components']
@@ -202,7 +202,9 @@ def lower_assignments(assignments, boundary_handling=None, function_name='kernel
     if data_type is not None:
         cdt = np.dtype({'double': np.float64, 'float': np.float32}.get(data_type, data_type))
     else:
-        cdt = np.result_type(*[f.dtype.numpy_dtype for f in input_fields + output_fields])
+        # bfloat16 computes in fp32 at least: np.result_type cannot promote the stand-in dtype
+        cdt = np.result_type(*[np.float32 if f.dtype.numpy_dtype == BFLOAT16 else f.dtype.numpy_dtype
+                               for f in input_fields + output_fields])
         if cdt.kind != 'f':
             cdt = np.dtype(np.float64)
         if cdt.itemsize < 4:

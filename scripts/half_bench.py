@@ -1,12 +1,17 @@
-"""float16 fields against the shipped precision, in one process on one GPU: forward and adjoint march kernels of C3, C2,
-C5 (fp32) and the 27-point stencil C4 (fp64) at their BASELINE shapes, each in float16 and in its own dtype, alternated.
+"""16-bit fields against the shipped precision, in one process on one GPU: forward and adjoint march kernels of C3, C2,
+C5 (fp32) and the 27-point stencil C4 (fp64) at their BASELINE shapes, each in float16, in bfloat16 and in its own dtype,
+alternated.
 
 Every timed region is 20 launches of one kernel, started from an idle GPU (a pause before it, like bench.py's
 cool-down: these B200s power-cap within ~150 ms of streaming), timed with CUDA events; the median over the repeats is
 reported per launch, with the achieved bandwidth from ``StencilKernelIR.bytes_per_cell`` (compulsory HBM bytes).  The
-accuracy of the float16 kernels is measured on sampled blocks against the fp64 oracle evaluated on the fp16 inputs
-converted exactly to fp64: max |got - ref| / max |ref| (DESIGN §6: <= 5e-4).  Card name and power limit are read in
-the same run.
+accuracy of the 16-bit kernels is measured on sampled blocks against the fp64 oracle evaluated on the 16-bit inputs
+converted exactly to fp64: max |got - ref| / max |ref| (DESIGN §6: <= 5e-4 for float16, <= 4e-3 for bfloat16).  Card
+name, power limit and max SM clock are read in the same run.
+
+Output per workload: ``speedup_forward`` / ``speedup_adjoint`` (float16 over the shipped dtype),
+``speedup_bf16_forward`` / ``speedup_bf16_adjoint`` (bfloat16 over the shipped dtype) and ``bf16_over_fp16_forward`` /
+``bf16_over_fp16_adjoint`` (float16 time / bfloat16 time: above 1 when bfloat16 is faster).
 
     python scripts/half_bench.py --out half_bench.json [--repeats 5] [--only c3,c4]"""
 import argparse
@@ -96,7 +101,8 @@ def run_workload(name, repeats, pause_s):
     shape, base = WORKLOADS[name]
     cells = int(np.prod(shape))
     legs = {}
-    for dt in ('float16', base):
+    dtypes = ('float16', 'bfloat16', base)
+    for dt in dtypes:
         op = make_config(name, shape=shape, dtype=dt, boundary_handling='zeros')
         tdt = getattr(torch, dt)
         tens = make_inputs(op, shape, tdt, seed=1)
@@ -115,7 +121,7 @@ def run_workload(name, repeats, pause_s):
         assert fwd.last_variant == 'march' and bwd.last_variant == 'march', (name, dt)
         legs[dt] = dict(op=op, fwd=fwd, bwd=bwd, fargs=fargs, bargs=bargs, tens=tens, ms_fwd=[], ms_bwd=[])
     for _ in range(repeats):
-        for dt in ('float16', base):
+        for dt in dtypes:
             L = legs[dt]
             L['ms_fwd'].append(time_kernel(L['fwd'], L['fargs'], pause_s))
             L['ms_bwd'].append(time_kernel(L['bwd'], L['bargs'], pause_s))
@@ -128,13 +134,16 @@ def run_workload(name, repeats, pause_s):
             row[which] = {'ms_median': round(ms, 4), 'ms_all': [round(v, 4) for v in L[key]], 'bytes_per_cell': bpc,
                           'achieved_TBps': round(bpc * cells / (ms * 1e-3) / 1e12, 3),
                           'kernel': (L['fwd'] if which == 'forward' else L['bwd']).last_instance}
-        if dt == 'float16':
+        if dt != base:
             # outputs of the last timed launches (inputs never change): checked on sampled blocks
             row['forward']['max_rel_err'] = sampled_error(name, shape, L['op'].forward_ast_gpu, L['tens'], 'forward')
             row['adjoint']['max_rel_err'] = sampled_error(name, shape, L['op'].backward_ast_gpu, L['tens'], 'backward')
         res[dt] = row
     for which in ('forward', 'adjoint'):
-        res['speedup_' + which] = round(res[base][which]['ms_median'] / res['float16'][which]['ms_median'], 3)
+        ms = {dt: res[dt][which]['ms_median'] for dt in dtypes}
+        res['speedup_' + which] = round(ms[base] / ms['float16'], 3)
+        res['speedup_bf16_' + which] = round(ms[base] / ms['bfloat16'], 3)
+        res['bf16_over_fp16_' + which] = round(ms['float16'] / ms['bfloat16'], 3)
     del legs
     torch.cuda.empty_cache()
     return res
