@@ -45,6 +45,14 @@ def main():
         asg, bh, shape, dtype = random_stencil(seed)
         op = ps.AutoDiffOp(asg, boundary_handling=bh, op_name='fuzz%d' % seed)
         kernels += [CompiledKernel(op.forward_ast_gpu), CompiledKernel(op.backward_ast_gpu)]
+    import test_gpu_fuzz16 as f16                               # tests/test_gpu_fuzz16.py
+    from stencil_fuzz import DOUBLE_SHAPES, fuzz_case
+    cases = [fuzz_case(seed, dtype) for seed in range(24) for dtype in ('float16', 'bfloat16')]
+    cases += [fuzz_case(seed, mixed=True) for seed in f16.MIXED_SEEDS]
+    for dtype, seed in f16.DOUBLE_CASES:
+        shape = DOUBLE_SHAPES[len(fuzz_case(seed, dtype)[3])]
+        cases.append(fuzz_case(seed, dtype, shape=shape, data_type='double'))
+    kernels += [CompiledKernel(ir) for case in cases for ir, _ in case[1]]
     for name, shape, dtype in (('c1', (20, 30), 'float32'), ('c1', (20, 32), 'float64'), ('c2', (96, 256), 'float32'),
                                ('c2', (33, 20), 'float64'), ('c3', (40, 48, 256), 'float32'), ('c4', (12, 20, 132), 'float64'),
                                ('c5', (3, 40, 136), 'float32')):       # tests/test_gpu_parity.py

@@ -157,6 +157,7 @@ def test_random_stencils_replay(seed):
             named[f.name] = a
         emu.run(ek, arrays)
         ref = evaluate(collection, {f.name: named[f.name].copy() for f in ir.input_fields}, bh)
+        assert all(np.count_nonzero(ref[f.name]) for f in ir.output_fields), (seed, 'empty interior')
         for f in ir.output_fields:
             scale = max(1.0, np.abs(ref[f.name]).max())
             assert np.isfinite(named[f.name]).all(), (seed, f.name)
