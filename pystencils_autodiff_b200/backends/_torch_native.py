@@ -93,10 +93,9 @@ class CompiledKernel:
                 raise ValueError('%s: two fused steps per launch are not available: %s' % (self.function_name, reason))
             self._emitted[variant] = emit_march_chain(self.ir, self.tuning_x2, peer=True)
         if variant == 'march_x2' and variant not in self._emitted:
-            reason = self.fused_steps_reason()
+            reason = self.fused_steps_reason()         # emits the pair when it can be built
             if reason:
                 raise ValueError('%s: two fused steps per launch are not available: %s' % (self.function_name, reason))
-            self._emitted[variant] = emit_march_chain(self._chain_ir(), self.tuning_x2)
         return self._emitted[variant]
 
     def _chain_ir(self):
@@ -105,10 +104,13 @@ class CompiledKernel:
             return lift_to_3d(self.ir)
         return self.ir
 
-    tuning_x2 = None   # MarchTuning of the fused-step kernel (None = emit_chain defaults)
+    tuning_x2 = None   # MarchTuning of the fused-step kernel (None = emit_chain defaults); set before the first use
 
     def fused_steps_reason(self):
-        """None when ``out = S(S(u))`` can run as one launch (emit_chain.py), else why not."""
+        """None when ``out = S(S(u))`` can run as one launch (emit_chain.py), else why not.  The answer is the emitter's:
+        the pair is emitted here (and kept), so that a stencil whose pair the tiling cannot hold — an x reach wider than a
+        thread's strip, a y halo taller than the tile, a staged box or ring too large — takes single steps wherever pairs
+        are the default instead of failing at its first launch."""
         try:
             return self._fused_reason          # asked per launch / per run() by the data handling: computed once
         except AttributeError:
@@ -116,7 +118,12 @@ class CompiledKernel:
         if self._components:
             reason = 'index dimensions'
         else:
-            reason = self._march_reason or chain_ineligible_reason(self._chain_ir())
+            reason = self._march_reason or chain_ineligible_reason(self._chain_ir(), self.tuning_x2)
+        if reason is None:
+            try:
+                self._emitted['march_x2'] = emit_march_chain(self._chain_ir(), self.tuning_x2)
+            except ValueError as e:
+                reason = str(e)
         self._fused_reason = reason
         return reason
 

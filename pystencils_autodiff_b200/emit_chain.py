@@ -42,7 +42,15 @@ from pystencils_autodiff_b200.linopt import plan_linear
 __all__ = ['chain_ineligible_reason', 'emit_march_chain']
 
 
-def chain_ineligible_reason(ir: StencilKernelIR) -> Optional[str]:
+def _strip_width(itemsize, tuning):
+    """Cells per thread along x (SX) of a fused-pair kernel."""
+    return (tuning.sx if tuning is not None else 0) or (4 if itemsize == 4 else 2)
+
+
+def chain_ineligible_reason(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None) -> Optional[str]:
+    """None when the stencil has the form a fused pair needs, else why not.  Geometry limits of a particular tiling
+    (tile height, TMA box, shared memory) are found by ``emit_march_chain`` itself; ask ``CompiledKernel.fused_steps_reason``
+    for the complete answer."""
     if any(f.dtype.numpy_dtype == np.dtype(np.float16) for f in ir.all_fields):
         # a pair would carry the intermediate field in fp32 and round once, two launches round it to fp16 in between
         return 'float16 fields: fused pairs not implemented'
@@ -62,6 +70,11 @@ def chain_ineligible_reason(ir: StencilKernelIR) -> Optional[str]:
         return 'input and output must have the same element type'
     if _planewise(ir.main[0][1]) is None:
         return 'a term couples several z planes'
+    # the x halo of a lane comes from its neighbour's strip (warp shuffle), so it cannot reach past one strip
+    reach_x = max(ir.halo(fin.name)[2])
+    sx = _strip_width(fin.dtype.itemsize, tuning)
+    if reach_x > sx:
+        return 'x reach of %d cells wider than the per-thread strip of %d cells' % (reach_x, sx)
     return None
 
 
@@ -75,7 +88,7 @@ def _planewise(rhs):
 
 def emit_march_chain(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, peer: bool = False) -> EmittedKernel:
     """Kernel computing ``out = S(S(u))`` for the single-step IR ``out = S(u)`` (fields: out, u)."""
-    reason = chain_ineligible_reason(ir)
+    reason = chain_ineligible_reason(ir, tuning)
     if reason:
         raise ValueError('fused-step march variant not applicable: ' + reason)
     t = tuning or MarchTuning()
@@ -105,7 +118,7 @@ def emit_march_chain(ir: StencilKernelIR, tuning: Optional[MarchTuning] = None, 
     if fp64_default:
         import dataclasses
         t = dataclasses.replace(t, ry=2, ty=18, sx=2, min_ctas=2)
-    SX = t.sx or (4 if es == 4 else 2)
+    SX = _strip_width(es, t)
     if (SX * es) % 16:
         raise ValueError('sx*itemsize must be a multiple of 16 bytes')
     if HXL > SX or HXR > SX:

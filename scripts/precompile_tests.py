@@ -53,6 +53,16 @@ def main():
         shape = DOUBLE_SHAPES[len(fuzz_case(seed, dtype)[3])]
         cases.append(fuzz_case(seed, dtype, shape=shape, data_type='double'))
     kernels += [CompiledKernel(ir) for case in cases for ir, _ in case[1]]
+    import test_gpu_fuzz_pairs as fp                            # tests/test_gpu_fuzz_pairs.py: pairs of both row modes
+    from stencil_fuzz import PAIR_SEEDS, pair_case
+    pair_kernels = [fp.pair_kernel(ir, tuning) for seed in PAIR_SEEDS for _, ir, _ in pair_case(seed)[0]
+                    for tuning in fp.ROW_MODES.values()]
+    for seed in fp.SLAB_SEEDS:
+        case, g = fp.slab_case(seed)
+        pair_kernels += [CompiledKernel(case[0][0][1]), fp.slab_local_kernel(seed, g)]
+    for k in pair_kernels:
+        k.fused_steps_reason()                                  # emits the pair where it can be built
+    kernels += pair_kernels
     for name, shape, dtype in (('c1', (20, 30), 'float32'), ('c1', (20, 32), 'float64'), ('c2', (96, 256), 'float32'),
                                ('c2', (33, 20), 'float64'), ('c3', (40, 48, 256), 'float32'), ('c4', (12, 20, 132), 'float64'),
                                ('c5', (3, 40, 136), 'float32')):       # tests/test_gpu_parity.py

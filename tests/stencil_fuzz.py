@@ -1,4 +1,5 @@
-"""Random stencil generator shared by the CPU (compile-only) and GPU (parity) fuzz tests, and the per-cell check of
+"""Random stencil generators shared by the CPU (compile-only / replay) and GPU (parity) fuzz tests — any stencil
+(``random_stencil``) and one-field stencils for fused pairs of steps (``random_pair_stencil``) — and the per-cell check of
 16-bit outputs against the fp64 oracle."""
 import random
 
@@ -6,6 +7,7 @@ import numpy as np
 import sympy as sp
 
 import pystencils_autodiff_b200 as ps
+from oracle.evaluate import evaluate
 
 # x extents for 2-byte fields, by the extent drawn for fp32 / fp64: 136 (a ragged second 128-cell tile), 264 and 40 give
 # 16-byte rows and take the march kernel; 36 (72-byte rows) takes the generic kernel only
@@ -73,6 +75,124 @@ def random_stencil(seed, shape=None, dtype=None, mixed=False):
     if new_shape != tuple(shape) or types != [drawn_dtype] * len(names):
         asg = retyped(asg, new_shape, dict(zip(names, types)))
     return ps.AssignmentCollection(asg), bh, new_shape, 'mixed' if mixed else (dtype or drawn_dtype)
+
+
+PAIR_SEEDS = range(32)
+# reach drawn per side: y / z up to 2, x up to 4 — fp32 strips are 4 cells (two radii beyond a strip need the pad-column
+# fix-up loads from 3 cells on), fp64 strips 2 (fix-up loads at 2 cells, no pair beyond)
+PAIR_REACH = {'z': (0, 1, 1, 2), 'y': (0, 1, 1, 2), 'x': (0, 1, 2, 2, 3, 4)}
+
+
+def random_pair_stencil(seed, shape=None):
+    """``(assignments, boundary_handling, shape, dtype, scalars)`` of random one-field stencil ``seed`` (``v = S(u)``) for
+    fused pairs of steps (emit_chain.py).
+
+    Every term touches one z plane: linear terms, products, ``exp``, ``sqrt`` and ``sin`` of accesses of one plane.  The
+    reach is drawn per axis and side (``PAIR_REACH``; one linear term sits at each drawn extreme, so the halo is exactly
+    the drawn one); sometimes with an access-free term, sometimes with a symbolic coefficient ``alpha`` whose value is in
+    ``scalars``.  2-D stencils have the 'zeros' boundary (the pair runs them lifted to one plane).  Shapes are ragged with
+    16-byte rows: y below and above one tile, x a few strips beyond one 120-column tile pitch, z below and above the
+    pair's warm-up of 2 x (z reach) planes.  With ``boundary_handling=None`` a drawn extent of at most twice the ghost
+    layers grows to ``2 * ghost_layers + 3``; a ``shape`` passed in is kept."""
+    rnd = random.Random('pair%d' % seed)
+    ndim = rnd.choice([2, 3, 3, 3])
+    dtype = rnd.choice(['float32', 'float64'])
+    bh = 'zeros' if ndim == 2 else rnd.choice(['zeros', None])
+    axes = 'zyx'[3 - ndim:]
+    reach = {a: (rnd.choice(PAIR_REACH[a]), rnd.choice(PAIR_REACH[a])) for a in axes}     # (low side, high side)
+    nonlinear = rnd.random() < 0.4
+    drawn_shape = tuple({'z': rnd.choice([2, 3, 11]), 'y': rnd.choice([13, 50]), 'x': rnd.choice([132, 136, 140])}[a]
+                        for a in axes)
+    drawn = shape is None
+    shape = drawn_shape if drawn else tuple(shape)
+    u, v = ps.fields('u, v: %s[%s]' % (dtype, ','.join(map(str, shape))))
+
+    def offset(**fixed):
+        return tuple(fixed[a] if a in fixed else rnd.randint(-reach[a][0], reach[a][1]) for a in axes)
+
+    def coeff():
+        return sp.Float(round(rnd.choice([-1, 1]) * rnd.uniform(0.2, 1.2), 3))
+
+    def plane_term(kind):
+        """A term whose accesses share one z plane."""
+        dz = {'z': rnd.randint(-reach['z'][0], reach['z'][1])} if ndim == 3 else {}
+
+        def access():
+            return u[offset(**dz)]
+        if kind == 'lin':
+            return coeff() * access()
+        if kind == 'prod':
+            return coeff() * access() * access()
+        if kind == 'exp':
+            return coeff() * sp.exp(-access() ** 2)
+        if kind == 'sqrt':
+            return coeff() * access() / sp.sqrt(access() ** 2 + 1)
+        return coeff() * sp.sin(access())
+
+    terms = []
+    for a in axes:                      # the drawn extremes
+        for side, r in zip((-1, 1), reach[a]):
+            if r:
+                terms.append(coeff() * u[offset(**{a: side * r})])
+    kinds = ['lin'] * rnd.randint(1, 3)
+    if nonlinear:
+        kinds += rnd.sample(['prod', 'exp', 'sqrt', 'sin'], rnd.randint(1, 2))
+    terms += [plane_term(k) for k in kinds]
+    rnd.shuffle(terms)
+    scalars = {}
+    if rnd.random() < 0.3:
+        # a symbolic coefficient of two terms, possibly of different planes: the sum splits by plane only once expanded
+        alpha = sp.Symbol('alpha')
+        scalars['alpha'] = round(rnd.uniform(0.3, 1.2), 3)
+        terms = [alpha * (terms[0] + terms[1])] + terms[2:] if len(terms) > 1 else [alpha * terms[0]]
+    if rnd.random() < 0.3:
+        terms.append(coeff())           # access-free
+    asg = {v.center: sp.Add(*terms)}
+    if bh is None and drawn:
+        gl = max(a.required_ghost_layers for a in asg[v.center].atoms(ps.Field.Access))
+        grown = tuple(2 * gl + 3 if n <= 2 * gl else n for n in shape)
+        if grown != shape:
+            asg, shape = retyped(asg, grown, dtype), grown
+    return ps.AssignmentCollection(asg), bh, shape, dtype, scalars
+
+
+# ---- one pair fuzz case (shared by the GPU test and its CPU replay) -----------------------------------------------------
+def pair_case(seed, shape=None):
+    """``(kernels, bh, shape, dtype, scalars)`` of ``random_pair_stencil(seed, shape)``; ``kernels``:
+    ``[(direction, ir, assignments)]`` of the forward and — where it reads the upstream gradient only (a linear stencil)
+    — the adjoint, the one-field kernels a pair can be asked of."""
+    asg, bh, shape, dtype, scalars = random_pair_stencil(seed, shape)
+    op = ps.AutoDiffOp(asg, boundary_handling=bh, op_name='pair%d' % seed)
+    kernels = [(d, ir, a) for d, ir, a in (('forward', op.forward_ast_gpu, op.forward_assignments),
+                                           ('adjoint', op.backward_ast_gpu, op.backward_assignments))
+               if len(ir.input_fields) == 1 and len(ir.output_fields) == 1]
+    return kernels, bh, shape, dtype, scalars
+
+
+def pair_input(shape, dtype, seed):
+    return np.random.default_rng(seed).uniform(-1, 1, size=shape).astype(dtype)
+
+
+def oracle_steps(assignments, ir, u, steps, bh, scalars):
+    """The fp64 oracle applied ``steps`` times to ``u``, every intermediate result cast to the field type (what a launch
+    per step stores); the last result in float64."""
+    fin, fout = ir.input_fields[0].name, ir.output_fields[0].name
+    r = u
+    for i in range(steps):
+        r = evaluate(assignments, {fin: r}, bh, scalars=scalars)[fout]
+        if i + 1 < steps:
+            r = r.astype(u.dtype)
+    return r
+
+
+def check_steps(got, ref, dtype, what=''):
+    """Every cell written (no NaN left from the prefilled output), finite, within the fuzz tolerance of the type."""
+    got = np.asarray(got, dtype=np.float64)
+    assert not np.isnan(got).any(), (what, 'cells not written', int(np.isnan(got).sum()))
+    assert np.count_nonzero(ref), (what, 'empty interior')
+    scale = max(1.0, np.abs(ref).max())
+    err = np.abs(got - ref).max()
+    assert np.isfinite(got).all() and err <= WIDE_TOL[dtype] * scale, (what, dtype, err, scale)
 
 
 def retyped(assignments, shape, types):
